@@ -1,7 +1,12 @@
-"""bench.py -- headline benchmark of the MOFA-Video hot path on B200 (contract: see the task prompt).
+"""bench.py -- headline benchmark of the MOFA-Video hot path on B200; prints one JSON result line.
 
     python bench.py --gpus N --steps K --warmup W            # engine arm (this repo's sm_100a path)
     python bench.py --impl reference --gpus N --steps K ...   # CPU arm: the oracle restatement of the reference
+    python bench.py ... --dump-outputs DIR                    # also save what the last timed clip computed
+
+--dump-outputs writes DIR/frames.npy: a fixed, seeded sample (float32) of the uint8 frames of the last timed clip, whose
+inputs and initial noise are seeded, so two builds run with the same arguments can be compared output for output.  Compare
+with a tolerance: two runs of one build on a B200 differed by 1 (of 255) in 5 % of the sampled values.
 
 Metric (BASELINE.json): frames/sec @ 576x1024x25f, 25 Euler steps.  One "step" of this benchmark is ONE CLIP
 through FlowControlNetPipeline.__call__ (CLIP embed + VAE encode + adapter cond branch + 25 x (adapter + UNet +
@@ -219,6 +224,23 @@ def _pin_to_gpu_numa_node(gpu_index):
 
 
 
+DUMP_SAMPLES = 1 << 23   # 32 MiB of float32; one 576x1024x25 clip is 44 M values (177 MB in float32)
+
+
+def _frames_sample(frames):
+    """A fixed, seeded sample of a clip's uint8 frames [T, H, W, 3] as float32: the same flat indices on every run."""
+    flat = frames.reshape(-1)
+    idx = torch.randperm(flat.numel(), generator=torch.Generator().manual_seed(0))[:DUMP_SAMPLES].sort().values
+    return flat[idx.to(flat.device)].float().cpu().numpy()
+
+
+def _write_dump(out_dir, arrays):
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
+
+
 def run_engine(args):
     import torch.distributed as dist
     from mofa_video_b200 import lib, parallel
@@ -321,18 +343,24 @@ def run_engine(args):
     if rank == 0:
         sampler.start()
     lib.launch_count_reset()
-    K = max(args.steps, 1)
+    K = args.steps
     if K > 1:
         ms_dev = timed(clip_device, K - 1)
     else:
         ms_dev = 0.0
-    # last timed clip: per-launch CUDA events for the roofline line
+    # last timed clip: per-launch CUDA events for the roofline line.  Its initial noise is re-seeded so that the frames
+    # --dump-outputs writes depend only on the seeds, not on how many clips --warmup / --steps ran before it.
     lib.profile_start()
-    ms_last = timed(clip_device, 1)
+    lat_gen.manual_seed(42 + rank)
+    last = []
+    ms_last = timed(lambda: last.append(clip_device()), 1)
     prof = lib.profile_stop()
     tim = pipe.last_timings_ms()
     ms_dev += ms_last
     launches = lib.launch_count()
+    # sampled now: later clips may reuse the pipeline's output buffer
+    dump = {"frames": _frames_sample(last[0].frames[0])} if args.dump_outputs and rank == 0 else None
+    del last
     if world > 1 and gather is None:  # NCCL communicator / buffers are created at the first collective: not timed
         parallel.gather_frames(torch.zeros(T, H, W, 3, dtype=torch.uint8, device=dev), dst=0)
         torch.cuda.synchronize()
@@ -397,6 +425,8 @@ def run_engine(args):
                        "d2h_bytes_per_step": int(d2h), "ms_per_step": round(ms_e2e / K, 2)},
                "gather": gather_kind, "host": {"cpus_pinned_to_gpu_numa_node": affinity, "cuda_graph_step": True},
                "gpu_launches": int(launches), "clocks": clocks}
+        if dump is not None:
+            _write_dump(args.dump_outputs, dump)
         print(json.dumps(out), flush=True)
     if world > 1:
         if gather is not None:
@@ -460,7 +490,13 @@ def main():
     ap.add_argument("--impl", default="engine", choices=["engine", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-other-configs", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write a seeded sample of the last timed clip's frames to DIR/frames.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl != "engine":
+        ap.error("--dump-outputs applies to the engine arm")
     if args.impl == "reference":
         run_reference(args)
     else:

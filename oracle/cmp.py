@@ -150,8 +150,9 @@ def cmp_demo_run(model, image, sparse, mask):
 
 
 def seeded_state_dict(model, seed=0):
-    """Deterministic weights for any module with CMP's key names (used for the reference-generated golden and for
-    the tests): N(0, 1/fan_in) convs, BN weight ~ U(0.5,1.5), bias/mean ~ N(0,0.1), var ~ U(0.5,1.5)."""
+    """Deterministic weights for any module with CMP-style key names (used for the reference-generated goldens of CMP
+    and of the adapter encoders, and for the tests): N(0, 1/fan_in) convs, norm weight ~ U(0.3,0.7), bias/mean ~
+    N(0,0.1), var ~ U(0.5,1.5)."""
     g = torch.Generator().manual_seed(seed)
     sd = {}
     for k, v in sorted(model.state_dict().items()):

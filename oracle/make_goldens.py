@@ -153,20 +153,20 @@ def make_adapter_encoders():
     spec = importlib.util.spec_from_file_location("ref_fcn", fn)
     m = importlib.util.module_from_spec(spec)
     spec.loader.exec_module(m)
-    torch.manual_seed(0)
+    from oracle.cmp import seeded_state_dict
     ce = m.FlowControlNetConditioningEmbeddingSVD(conditioning_embedding_channels=32)   # small: keeps the fixture < 1 MB
     fe = m.FlowControlNetFirstFrameEncoder(c_in=32, channels=[32, 64, 128])
+    # seeded weights (no zero-convs left, so the fixture exercises them) are rebuilt by the test from the seeds:
+    # only inputs and outputs are stored
+    ce.load_state_dict(seeded_state_dict(ce, seed=11))
+    fe.load_state_dict(seeded_state_dict(fe, seed=12))
     gen = torch.Generator().manual_seed(1)
     with torch.no_grad():
-        for mod in (ce, fe):  # un-zero the zero-convs so the fixture exercises them
-            for p in mod.parameters():
-                if p.abs().max() == 0:
-                    p.copy_(torch.randn(p.shape, generator=gen) * 0.02)
         cond_in = torch.randn(1, 3, 64, 64, generator=gen)
         cond_out = ce(cond_in)
         flow_out = fe(cond_out)
-    g = {"cond_embedding_sd": ce.state_dict(), "flow_encoder_sd": fe.state_dict(), "cond_in": cond_in,
-         "cond_out": cond_out, "flow_out": flow_out}
+    g = {"cond_embedding_seed": 11, "flow_encoder_seed": 12, "cond_in": cond_in, "cond_out": cond_out,
+         "flow_out": flow_out}
     torch.save(g, os.path.join(OUT, "adapter_encoders.pt"))
     print("adapter encoder golden written:", [tuple(t.shape) for t in flow_out])
 
@@ -223,7 +223,10 @@ def make_cmp():
         py = F.softmax(logits[:, nb:], dim=1) * mesh
         flow = torch.cat([px.sum(1, keepdim=True), py.sum(1, keepdim=True)], dim=1)
         flow_up = F.interpolate(flow, size=(128, 128), mode="bilinear", align_corners=True)
-    torch.save({"image": image, "sparse": sparse, "mask": mask, "logits_sub": logits[:, ::9, ::4, ::4].clone(),
+    # the hints as (batch, y, x) points and their flow values: the dense sparse / mask tensors are rebuilt from them
+    points = mask[:, 0].nonzero()
+    values = sparse[points[:, 0], :, points[:, 1], points[:, 2]]
+    torch.save({"image": image, "points": points, "values": values, "logits_sub": logits[:, ::9, ::4, ::4].clone(),
                 "flow": flow_up, "seed": 3}, os.path.join(OUT, "cmp_small.pt"))
     print("cmp golden written:", tuple(logits.shape), float(flow_up.abs().mean()))
 
@@ -836,10 +839,77 @@ def make_sparse_flow():
     print("sparse-flow golden written:", {k: tuple(v.shape) for k, v in out.items()})
 
 
+def make_init_models_calls():
+    """tests/golden/init_models_calls.json: every call the reference's model-loading function `init_models`
+    (MOFA-Video-Traj/run_gradio.py:90-159, extracted verbatim) makes on the names it imports, in order, recorded by
+    running it against recording stand-ins with its default options.  tests/test_boundary_init_models_cpu.py replays the
+    calls against this package.  Encoding: {"ref": n} is the object op n returned, {"arg": name} an argument of
+    init_models, anything else a literal."""
+    import json
+    ops = []
+
+    def enc(v):
+        if isinstance(v, _Rec):
+            return {"ref": v.ref}
+        if isinstance(v, _Arg):
+            return {"arg": v.name}
+        if isinstance(v, (tuple, list)):
+            return [enc(x) for x in v]
+        assert v is None or isinstance(v, (str, int, float, bool)), type(v)
+        return v
+
+    class _Arg:
+        def __init__(self, name):
+            self.name = name
+
+    class _Rec:
+        def __init__(self, op):
+            ops.append({**op, "out": len(ops)})
+            self.ref = len(ops) - 1
+
+        def __getattr__(self, method):
+            if method.startswith("__"):
+                raise AttributeError(method)
+            return lambda *a, **k: _Rec({"op": "call", "obj": self.ref, "method": method, "args": enc(a),
+                                         "kwargs": {n: enc(v) for n, v in k.items()}})
+
+        def __call__(self, *a, **k):
+            return _Rec({"op": "call", "obj": self.ref, "method": None, "args": enc(a),
+                         "kwargs": {n: enc(v) for n, v in k.items()}})
+
+    def module(name):
+        m = _mod(name)
+
+        def getattr_(attr):        # the import machinery probes dunders and looks a name up more than once
+            if attr.startswith("__"):
+                raise AttributeError(attr)
+            rec = _Rec({"op": "name", "module": name, "name": attr})
+            setattr(m, attr, rec)
+            return rec
+        m.__getattr__ = getattr_
+        return m
+
+    for name in ("models", "pipeline", "models.unet_spatio_temporal_condition_controlnet", "pipeline.pipeline",
+                 "models.svdxt_featureflow_forward_controlnet_s2d_fixcmp_norefine"):
+        module(name)
+    ns = {n: _Rec({"op": "name", "module": None, "name": n})
+          for n in ("CLIPVisionModelWithProjection", "AutoencoderKLTemporalDecoder")}
+    _extract_functions(os.path.join(REF, "run_gradio.py"), ["init_models"], ns)
+    args = ("pretrained_model_name_or_path", "resume_from_checkpoint", "weight_dtype", "device")
+    ret = ns["init_models"](*[_Arg(a) for a in args])
+    out ={"args": list(args), "ops": ops, "returns": enc(ret)}
+    with open(os.path.join(OUT, "init_models_calls.json"), "w") as f:
+        json.dump(out, f, indent=1)
+    print("init_models call trace written:", len(ops), "ops")
+
+
 if __name__ == "__main__":
     os.makedirs(OUT, exist_ok=True)
     if "--sparse-flow" in sys.argv:
         make_sparse_flow()
+        sys.exit(0)
+    if "--init-models" in sys.argv:
+        make_init_models_calls()
         sys.exit(0)
     make_scheduler()
     if "--networks" in sys.argv or "--all" in sys.argv:

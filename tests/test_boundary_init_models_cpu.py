@@ -1,15 +1,16 @@
 """-m "not gpu": the drop-in boundary as the reference's own script reaches it (SURVEY.md §8b, §3.5).
 
-`init_models` is taken VERBATIM (ast) out of /root/reference/MOFA-Video-Traj/run_gradio.py:90-159 and executed against
-this package: its `from models... import`, `from pipeline.pipeline import` lines resolve to mofa_video_b200/ (first on
-sys.path, INTEGRATION.md), `CLIPVisionModelWithProjection` / `AutoencoderKLTemporalDecoder` (transformers / diffusers
-loaders, absent here) are stand-ins that read the same checkpoint folders, and the checkpoint tree is synthetic but laid
-out per /root/reference/MOFA-Video-Hybrid/ckpt_tree.md:60-84.  Checks: the function runs unmodified; the VAE it hands
-over (an AutoencoderKLTemporalDecoder-layout nn.Module) is re-hosted on the engine, so decode does not fall to eager
-PyTorch; a clip through the resulting pipeline matches the oracle.  Also `FlowControlNet.from_unet`
-(models/controlnet_sdv.py:572-628).  CPU backend = tests/ref_ops.py via models._base.default_backend.
-Skipped where /root/reference is absent (the GPU box)."""
-import ast
+tests/golden/init_models_calls.json records every call the reference's `init_models` (MOFA-Video-Traj/run_gradio.py:
+90-159) makes on the names it imports, in order (oracle/make_goldens.py --init-models ran the function itself against
+recording stand-ins).  The test replays those calls against this package: its `from models... import`,
+`from pipeline.pipeline import` names resolve to mofa_video_b200/ (first on sys.path, INTEGRATION.md),
+`CLIPVisionModelWithProjection` / `AutoencoderKLTemporalDecoder` (transformers / diffusers loaders, absent here) are
+stand-ins that read the same checkpoint folders, and the checkpoint tree is synthetic but laid out per the reference's
+MOFA-Video-Hybrid/ckpt_tree.md:60-84.  Checks: the calls run unmodified; the VAE they hand over (an
+AutoencoderKLTemporalDecoder-layout nn.Module) is re-hosted on the engine, so decode does not fall to eager PyTorch; a
+clip through the resulting pipeline matches the oracle.  Also `FlowControlNet.from_unet` (models/controlnet_sdv.py:
+572-628).  CPU backend = tests/ref_ops.py via models._base.default_backend."""
+import importlib
 import json
 import os
 import sys
@@ -26,9 +27,8 @@ from oracle import fixtures
 from oracle import pipeline as opipe
 from oracle import scheduler as osched
 
-REF_SCRIPT = "/root/reference/MOFA-Video-Traj/run_gradio.py"
+CALLS = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "init_models_calls.json")
 PKG = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "mofa_video_b200")
-pytestmark = pytest.mark.skipif(not os.path.exists(REF_SCRIPT), reason="needs /root/reference (builder container)")
 
 
 def _write_model(d, cfg, sd, name):
@@ -122,22 +122,35 @@ def _loader_stubs(cfg):
     return CLIPVisionModelWithProjection, AutoencoderKLTemporalDecoder
 
 
-def _extract_init_models():
-    with open(REF_SCRIPT) as f:
-        tree = ast.parse(f.read())
-    fn = [n for n in tree.body if isinstance(n, ast.FunctionDef) and n.name == "init_models"]
-    assert len(fn) == 1
-    return compile(ast.Module(body=fn, type_ignores=[]), REF_SCRIPT, "exec")
+def _replay_init_models(names, *args):
+    """Run the recorded calls of the reference's init_models(*args); `names` answers its non-package imports."""
+    with open(CALLS) as f:
+        rec = json.load(f)
+    argv = dict(zip(rec["args"], args))
+    objs = {}
+
+    def dec(v):
+        if isinstance(v, list):
+            return [dec(x) for x in v]
+        if isinstance(v, dict):
+            return objs[v["ref"]] if "ref" in v else argv[v["arg"]]
+        return v
+
+    for op in rec["ops"]:
+        if op["op"] == "name":
+            obj = names[op["name"]] if op["module"] is None else getattr(importlib.import_module(op["module"]), op["name"])
+        else:
+            fn = objs[op["obj"]] if op["method"] is None else getattr(objs[op["obj"]], op["method"])
+            obj = fn(*dec(op["args"]), **{k: dec(v) for k, v in op["kwargs"].items()})
+        objs[op["out"]] = obj
+    return tuple(dec(rec["returns"]))
 
 
 def test_reference_init_models_runs_unmodified_against_the_shim(tmp_path, monkeypatch):
     cfg = dict(fixtures.TINY_CONFIG)
     svd, ctrl, unet, adapter, vae, clip = _checkpoint_tree(str(tmp_path), cfg)
     clip_cls, vae_cls = _loader_stubs(cfg)
-    from packaging import version
-    ns = {"CLIPVisionModelWithProjection": clip_cls, "AutoencoderKLTemporalDecoder": vae_cls, "torch": torch,
-          "version": version, "is_xformers_available": lambda: False}
-    exec(_extract_init_models(), ns)
+    names = {"CLIPVisionModelWithProjection": clip_cls, "AutoencoderKLTemporalDecoder": vae_cls}
     monkeypatch.chdir(tmp_path)
     monkeypatch.syspath_prepend(PKG)                      # INTEGRATION.md: mofa_video_b200/ first on sys.path
     saved = {k: sys.modules.pop(k) for k in list(sys.modules) if k.split(".")[0] in ("models", "pipeline", "utils")}
@@ -145,7 +158,7 @@ def test_reference_init_models_runs_unmodified_against_the_shim(tmp_path, monkey
         with _base.default_backend(ref_ops, "cpu"):
             # weight_dtype: the script passes torch.float16 on its CUDA device (run_gradio.py:223); the third-party CLIP /
             # VAE stand-ins stay fp32 on this CPU backend, the engine models accept only fp16 (checked below)
-            pipeline, cmp = ns["init_models"](svd, ctrl, weight_dtype=None, device="cpu")
+            pipeline, cmp = _replay_init_models(names, svd, ctrl, None, "cpu")
             assert type(pipeline).__module__ == "pipeline.pipeline" and type(pipeline.unet).__module__.startswith("models.")
             with pytest.raises(ValueError):
                 pipeline.unet.to("cpu", dtype=torch.float32)

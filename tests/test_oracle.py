@@ -10,6 +10,7 @@ from oracle import scheduler as osched
 from oracle.softsplat import softsplat
 
 GOLD = os.path.join(os.path.dirname(__file__), "golden")
+FIXTURE_THREADS = 8   # torch intra-op threads of the host that generated the pipeline fixtures
 
 
 def _gold(name):
@@ -55,12 +56,13 @@ def test_product_scheduler_matches_reference_fixture():
 
 
 def test_adapter_encoders_match_reference_fixture():
+    from oracle.cmp import seeded_state_dict
     from oracle.models import FlowControlNetConditioningEmbeddingSVD, FlowControlNetFirstFrameEncoder
     g = _gold("adapter_encoders.pt")
     ce = FlowControlNetConditioningEmbeddingSVD(32)
-    ce.load_state_dict(g["cond_embedding_sd"])
+    ce.load_state_dict(seeded_state_dict(ce, seed=g["cond_embedding_seed"]))
     fe = FlowControlNetFirstFrameEncoder(c_in=32, channels=(32, 64, 128))
-    fe.load_state_dict(g["flow_encoder_sd"])
+    fe.load_state_dict(seeded_state_dict(fe, seed=g["flow_encoder_seed"]))
     with torch.no_grad():
         c = ce(g["cond_in"])
         assert torch.allclose(c, g["cond_out"], rtol=1e-5, atol=1e-6)
@@ -138,7 +140,10 @@ def test_pipeline_call_matches_reference_fixture(fixture):
     UNet / FlowControlNet / scheduler files; DiffusionPipeline and VaeImageProcessor stubbed, oracle/make_goldens.py:
     make_pipeline).  oracle.pipeline.run_pipeline -- the oracle every engine pipeline test compares against -- must
     reproduce the 2-step latents: PIL conversion, CLIP resize path (Q3), VAE encode of the noise-augmented frame (Q7),
-    added-time-id constants (Q4), CFG with the per-frame scale, Karras-sigma Euler steps."""
+    added-time-id constants (Q4), CFG with the per-frame scale, Karras-sigma Euler steps.
+
+    Runs with the FIXTURE_THREADS intra-op threads the fixtures were generated with: the square clip's latents move by
+    ~7e-5 of their max when the CPU reductions are split across another thread count (3 or 16), beyond the 1e-5 below."""
     import PIL.Image
 
     from oracle import pipeline as opipe
@@ -151,20 +156,25 @@ def test_pipeline_call_matches_reference_fixture(fixture):
     pil = PIL.Image.fromarray(g["image_u8"].numpy())
     flow = fixtures.make_flow(T, H, W)
     lat0 = torch.randn(1, T, 4, H // 8, W // 8, generator=torch.Generator().manual_seed(g["latent_seed"]))
-    out = opipe.run_pipeline(vae, clip, unet, ad, osched.EulerDiscreteScheduler(), pil, pil, flow, height=H, width=W,
-                             num_inference_steps=g["steps"], latents=lat0.clone(),
-                             generator=torch.Generator().manual_seed(g["generator_seed"]), output_type="latent",
-                             controlnet_cond_scale=g["cond_scale"])
+    threads = torch.get_num_threads()
+    torch.set_num_threads(FIXTURE_THREADS)
+    try:
+        out = opipe.run_pipeline(vae, clip, unet, ad, osched.EulerDiscreteScheduler(), pil, pil, flow, height=H, width=W,
+                                 num_inference_steps=g["steps"], latents=lat0.clone(),
+                                 generator=torch.Generator().manual_seed(g["generator_seed"]), output_type="latent",
+                                 controlnet_cond_scale=g["cond_scale"])
+    finally:
+        torch.set_num_threads(threads)
     assert out.shape == g["latents"].shape
     assert (out - g["latents"]).abs().max().item() <= 1e-5 * g["latents"].abs().max().item()
 
 
 def test_adapter_parameter_names_match_the_reference_training_dump():
-    """/root/reference/Training/rec_para_train.txt is the reference's own dump of `controlnet.named_parameters()` names
+    """The reference's Training/rec_para_train.txt is its own dump of `controlnet.named_parameters()` names
     (train_stage1.py:846-856) -- 683 names produced by the REAL diffusers 0.24 blocks.  The oracle adapter (hence
     oracle/d24_blocks.py's module structure: resnets / attentions / transformer_blocks / temporal blocks / mixers) must
-    have exactly that name set.  Compared through a digest so no reference file is copied:
-    sha256 of the sorted names joined by newlines (regenerate: see the two lines below with the reference mounted)."""
+    have exactly that name set.  Compared through a digest of that file so no reference file is copied:
+    sha256 of its sorted non-empty lines joined by newlines."""
     import hashlib
     from oracle.models import FlowControlNet
     with torch.device("meta"):
@@ -172,10 +182,6 @@ def test_adapter_parameter_names_match_the_reference_training_dump():
     assert len(names) == 683
     digest = hashlib.sha256("\n".join(names).encode()).hexdigest()
     assert digest == "dde7b69aad4901bc3ef3bcd4f1301973a7749dd83d6f843e466b3b599d358dd5"
-    ref_file = "/root/reference/Training/rec_para_train.txt"
-    if os.path.exists(ref_file):  # builder container only: check the digest against the file itself
-        ref = sorted(line.strip() for line in open(ref_file) if line.strip())
-        assert hashlib.sha256("\n".join(ref).encode()).hexdigest() == digest
 
 
 def test_softsplat_oracle_matches_reference_kernel_golden():

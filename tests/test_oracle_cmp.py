@@ -13,11 +13,15 @@ GOLD = os.path.join(os.path.dirname(__file__), "golden", "cmp_small.pt")
 @pytest.mark.skipif(not os.path.exists(GOLD), reason="golden not generated")
 def test_cmp_oracle_matches_reference_fixture():
     g = torch.load(GOLD)
+    b, y, x = g["points"].unbind(1)
+    sparse = torch.zeros(g["image"].shape[0], 2, *g["image"].shape[2:])
+    mask = torch.zeros_like(sparse)
+    sparse[b, :, y, x], mask[b, :, y, x] = g["values"], 1.0
     m = ocmp.CMP().eval()
     m.load_state_dict(ocmp.seeded_state_dict(m, seed=g["seed"]))
     with torch.no_grad():
-        logits = m(g["image"] * 2 - 1, torch.cat([g["sparse"], g["mask"]], 1))
-        flow = ocmp.cmp_demo_run(m, g["image"], g["sparse"], g["mask"])
+        logits = m(g["image"] * 2 - 1, torch.cat([sparse, mask], 1))
+        flow = ocmp.cmp_demo_run(m, g["image"], sparse, mask)
     assert torch.allclose(logits[:, ::9, ::4, ::4], g["logits_sub"], rtol=1e-5, atol=1e-5)
     assert torch.allclose(flow, g["flow"], rtol=1e-5, atol=1e-4)
 

@@ -5,8 +5,9 @@ tests/golden/softsplat_ref.pt holds outputs of the reference's own CUDA-C `softs
 compiled with nvcc and launched on a B200, then normalised by the reference's own `softsplat(..., 'avg')` wrapper
 (recipe: oracle/make_softsplat_ref.py).  Here: `mofa_softsplat_avg` through the reference-signature entry point
 models.softsplat.softsplat must reproduce it (fp16 feature storage: <= 2e-3 * max|ref| + 1e-3), on collisions,
-out-of-bounds targets, non-finite flow, zero flow and integer shifts.  When oracle/_ref/libsoftsplat_ref.so travelled
-to this box, the reference kernel is also re-run live against oracle/softsplat.py (fp32 atomics: <= 1e-5)."""
+out-of-bounds targets, non-finite flow, zero flow and integer shifts.  The reference kernel's raw outputs are also held
+against oracle/softsplat.py (fp32 atomics: <= 1e-5): re-run live when oracle/_ref/libsoftsplat_ref.so was built,
+otherwise as recorded in the fixture."""
 import os
 
 import pytest
@@ -32,11 +33,13 @@ def test_engine_softsplat_matches_reference_kernel_golden():
         assert err <= tol, f"case {i} ({gold['kinds'][i]}): {err} > {tol}"
 
 
-@pytest.mark.skipif(not os.path.exists(ref.LIB), reason="oracle/_ref/libsoftsplat_ref.so not built (builder container only)")
 def test_reference_kernel_live_vs_oracle():
+    """The reference kernel is re-run when oracle/_ref/libsoftsplat_ref.so was built (it needs the reference's source);
+    otherwise its raw outputs recorded in tests/golden/softsplat_ref.pt on the same seeded inputs stand in."""
+    gold = None if os.path.exists(ref.LIB) else torch.load(ref.GOLDEN)
     for i in range(len(ref.CASES)):
         x, fl = ref.make_case(i)
-        raw = ref.run_reference_kernel(i, x, fl)
+        raw = ref.run_reference_kernel(i, x, fl) if gold is None else gold["cases"][i]["out_sum"]
         ones = torch.cat([x, x.new_ones(x.shape[0], 1, x.shape[2], x.shape[3])], 1)
         want = oracle_softsplat_out(ones, fl)
         assert (raw - want).abs().max().item() <= 1e-5 * max(1.0, want.abs().max().item()), i
